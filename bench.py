@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path (libbarvae.so)
     python bench.py --impl reference --gpus N --steps K ...   # the reference algorithm on the host CPU cores
+    python bench.py ... --dump-outputs DIR                    # also write the last timed step's loss (.npy)
 
 A "step" is one pass of the hot path over one batch of synthetic piano-roll bars: zero_grad, generator forward
 (phrase encoder, encoder x2, decoder), BCE loss, backward, (NCCL gradient all-reduce), Adam -- the pre-training
@@ -102,6 +103,18 @@ def synthetic_batch(B, seed, device, pin=False):
     if device is not None:
         return tuple(t.to(device) for t in ts)
     return tuple(t.pin_memory() for t in ts) if pin else ts
+
+
+def dump_outputs(out_dir, loss):
+    """--dump-outputs: what the last timed training step returns to its caller -- its loss -- as DIR/loss.npy (float32).
+    The gradients and updated parameters it leaves in the model are not written: with the reference's N(-1,1)
+    initialisation the step is so ill-conditioned that the order of the fp32 atomic additions in the InstanceNorm
+    statistics and the norm-block backward decides them (measured on one B200, 10 timed steps after 3 warm-up steps: two
+    runs' sampled gradients differ by 112 % rel-Frobenius, and the loss itself by 0.4-1.9 %), so they cannot be compared
+    between builds; the loss is the only value of the step a caller receives."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "loss.npy"), loss.detach().float().reshape(1).cpu().numpy())
 
 
 def cpu_reference_arm(batch, steps, warmup, target_s=0.0):
@@ -371,7 +384,14 @@ def main():
     ap.add_argument("--no-decode", action="store_true", help="train mode: skip the extra.decode measurement")
     ap.add_argument("--no-eager", action="store_true", help="train mode: skip extra.torch_eager_gpu")
     ap.add_argument("--eager-bars", type=int, default=256, help="bars per step of the PyTorch-eager comparator")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="train mode: after the timed steps, write the loss the last timed step returned as DIR/loss.npy "
+                         "(see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be >= 1 and --warmup >= 0")
+    if args.dump_outputs and (args.mode != "train" or args.impl != "barvae"):
+        ap.error("--dump-outputs applies to the training step of this repo's CUDA path (--mode train --impl barvae)")
 
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -466,8 +486,10 @@ def _train_bench(args, pkg, eng, par, Model, trainer, model, flat, reducer, cfg,
             ms = float(t)
         return ms
 
+    last_loss = [None]
+
     def step_resident():
-        trainer.step(*dbatch)
+        last_loss[0] = trainer.step(*dbatch)
 
     def step_e2e():
         loss = trainer.step_from_host(*hbatch)      # pinned host tensors -> H2D copies -> step, strictly in sequence
@@ -495,6 +517,8 @@ def _train_bench(args, pkg, eng, par, Model, trainer, model, flat, reducer, cfg,
     launches = pkg.launch_count()
     clocks = sampler.stop() if rank == 0 else None
     value = B * world * args.steps / (ms * 1e-3)
+    if args.dump_outputs and rank == 0:          # before the e2e loops below train the model further
+        dump_outputs(args.dump_outputs, last_loss[0])
 
     loop_e2e(hbatch, 2)
     ms_e2e = timed(lambda: loop_e2e(hbatch, args.steps), 1)

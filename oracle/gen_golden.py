@@ -3,7 +3,7 @@
 
 TEST INFRASTRUCTURE.  Run in the build container only (needs /root/reference):
 
-    python oracle/gen_golden.py            # writes tests/golden/golden_v1.pt
+    python oracle/gen_golden.py            # writes tests/golden/golden_v1.<i>.pt (oracle/golden_io.py)
 
 The reference has no tests or golden vectors of its own (SURVEY.md section 4), so these
 vectors -- outputs of the reference's own ``graph.*`` classes on seeded inputs and on
@@ -31,6 +31,7 @@ sys.path.insert(0, HERE)
 sys.path.insert(0, REF)
 
 import barvae_oracle as O  # noqa: E402
+from golden_io import save_golden  # noqa: E402
 
 torch.set_num_threads(8)
 
@@ -244,10 +245,8 @@ def main():
     G["sample"] = {"seed_w": 11, "latents": latents, "roll": torch.cat(outputs, 0).to(torch.uint8),
                    "first_probs": first_probs, "music_length": music_length}
 
-    out = os.path.join(HERE, "..", "tests", "golden", "golden_v1.pt")
-    os.makedirs(os.path.dirname(out), exist_ok=True)
-    torch.save(G, out)
-    print("wrote %s (%.1f KB) in %.1fs" % (out, os.path.getsize(out) / 1024, time.time() - t0))
+    save_golden(G, "golden_v1")
+    print("wrote tests/golden/golden_v1.*.pt in %.1fs" % (time.time() - t0))
 
 
 if __name__ == "__main__":

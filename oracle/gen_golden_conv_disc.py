@@ -1,5 +1,5 @@
 #!/usr/bin/env python
-"""Generate tests/golden/golden_conv_disc_v1.pt by running the reference's convolutional BarDiscriminator (UNMODIFIED) and
+"""Generate tests/golden/golden_conv_disc_v1.<i>.pt by running the reference's convolutional BarDiscriminator (UNMODIFIED) and
 its Refiner on CPU.  TEST INFRASTRUCTURE; build container only (needs /root/reference):
 
     python oracle/gen_golden_conv_disc.py
@@ -21,6 +21,7 @@ sys.path.insert(0, REF)
 
 import barvae_oracle as O  # noqa: E402
 import disc_oracle as D  # noqa: E402
+from golden_io import save_golden  # noqa: E402
 
 torch.set_num_threads(8)
 
@@ -77,9 +78,8 @@ def main():
         sd = D.make_conv_state_dict(rspec, seed, kind)
         G["refiner/%s/train" % kind] = run(ref, sd, xr, True, target_ones=False)
         G["refiner/%s/eval" % kind] = run(ref, sd, xr, False, target_ones=False)
-    out = os.path.join(os.path.dirname(HERE), "tests", "golden", "golden_conv_disc_v1.pt")
-    torch.save(G, out)
-    print("wrote", out, os.path.getsize(out), "bytes")
+    save_golden(G, "golden_conv_disc_v1")
+    print("wrote tests/golden/golden_conv_disc_v1.*.pt")
 
 
 if __name__ == "__main__":

@@ -18,7 +18,8 @@ def pytest_configure(config):
 
 @pytest.fixture(scope="session")
 def golden():
-    return torch.load(os.path.join(ROOT, "tests", "golden", "golden_v1.pt"), map_location="cpu", weights_only=False)
+    from golden_io import load_golden
+    return load_golden("golden_v1")
 
 
 @pytest.fixture(scope="session")

@@ -18,6 +18,16 @@ def test_stdout_carries_only_the_json_line():
     assert "NCCL version banner" in r.stderr and "python-level chatter" in r.stderr
 
 
+def test_arguments_it_cannot_honour_are_refused():
+    """--steps sets the number of timed steps, so no step count below one is silently raised; --dump-outputs is the
+    training step's"""
+    bench = os.path.join(ROOT, "bench.py")
+    for extra in (["--steps", "0"], ["--warmup", "-1"], ["--mode", "decode", "--dump-outputs", "out"],
+                  ["--impl", "reference", "--dump-outputs", "out"]):
+        r = subprocess.run([sys.executable, bench] + extra, capture_output=True, text=True, timeout=120)
+        assert r.returncode == 2 and r.stdout == "" and "error" in r.stderr, (extra, r.stderr[-500:])
+
+
 def test_reference_arm_line_has_the_contract_keys():
     """--impl reference: the oracle port on the host cores, same metric / config keys as the CUDA arm (tiny sample)"""
     r = subprocess.run([sys.executable, os.path.join(ROOT, "bench.py"), "--impl", "reference", "--steps", "1",

@@ -7,6 +7,7 @@ import pytest
 import torch
 import torch.nn.functional as F
 
+from golden_io import load_golden
 from gpu_util import ROOT, pkg
 
 
@@ -73,7 +74,7 @@ def test_discriminator_mirrors_keep_reference_keys_and_refuse_cpu():
 
 @pytest.fixture(scope="module")
 def gc():
-    return torch.load(os.path.join(ROOT, "tests", "golden", "golden_conv_disc_v1.pt"), map_location="cpu", weights_only=False)
+    return load_golden("golden_conv_disc_v1")
 
 
 def _run_conv(fwd, spec, seed, kind, x, training, D, target_ones):

@@ -9,21 +9,21 @@ rel-Frobenius against the oracle evaluated at the storage precision (measured: 2
 in eval mode; values go to gpurun_out/parity_report.jsonl);
 BatchNorm running statistics after the call 2e-3.  Reference-init weights (N(-1,1) everywhere, BatchNorm gammas included):
 forward only."""
-import os
 from collections import OrderedDict
 
 import pytest
 import torch
 import torch.nn.functional as F
 
-from gpu_util import ROOT, pkg, rel_fro, report
+from golden_io import load_golden
+from gpu_util import pkg, rel_fro, report
 
 pytestmark = pytest.mark.gpu
 
 
 @pytest.fixture(scope="module")
 def gc():
-    return torch.load(os.path.join(ROOT, "tests", "golden", "golden_conv_disc_v1.pt"), map_location="cpu", weights_only=False)
+    return load_golden("golden_conv_disc_v1")
 
 
 class _Storage:

@@ -1,5 +1,5 @@
 """CPU: pin the oracle restatement (oracle/barvae_oracle.py) to outputs of the reference itself
-(tests/golden/golden_v1.pt, produced by oracle/gen_golden.py from /root/reference)."""
+(tests/golden/golden_v1.<i>.pt, produced by oracle/gen_golden.py from the reference's own modules)."""
 from collections import OrderedDict
 
 import pytest
