@@ -280,6 +280,21 @@ int bvae_unpack_bits(const void* bits, int64_t nbits, void* out_bf16, float* out
 int bvae_threshold_pack(const float* p, int64_t n, float threshold, void* bits, float* out_f32, void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------
+ * Bernoulli draw per piano-roll cell with temperature, from a counter-based stream (the torch.gt(., 0.3) of
+ * maker_bar.py:39 replaced by a draw):
+ *   p = 1.f / (1.f + expf(-(logit * inv_temperature))),  cell = (u < p) ? 1 : 0,  u = (float)(r >> 8) * 2^-24,
+ *   r = word (i % 4) of Philox4x32-10(counter = {i / 4, bar_index, song lo32, song hi32}, key = {seed lo32, seed hi32}),
+ *   i = cell index in the bar (0..5759, C order [96][60]), song = song_base + b for bar row b of `logits`.
+ * A cell's draw depends only on (seed, song, bar_index, i): not on the batch size or the split of songs across calls.
+ * p is fit_sigmoid_fwd's expression, so at inv_temperature 1 it equals the decoder's probability bit for bit.
+ * A NaN logit gives 0, +inf gives 1, -inf gives 0.  inv_temperature finite and > 0 and bars >= 0, else
+ * BVAE_ERR_SHAPE; logits and out_f32 16-byte aligned, else BVAE_ERR_ALIGN.
+ * ------------------------------------------------------------------------------------------------------------ */
+int bvae_bernoulli_sample(const float* logits /* [bars][5760] */, int64_t bars, float inv_temperature,
+                          uint64_t seed, int64_t song_base, int32_t bar_index,
+                          float* out_f32 /* [bars][5760] {0,1} */, void* stream);
+
+/* ------------------------------------------------------------------------------------------------------------
  * nn.BatchNorm2d(C, eps, momentum, affine) (+ optional (Leaky)ReLU) on an NHWC tensor with few channels: the norm of the
  * GAN-phase piano-roll discriminator (graph/bar_discriminator.py:19-23,69,113-114,153: BatchNorm2d(8..64, eps=1e-5,
  * momentum=0.01), OnOffFeature's default-momentum BatchNorm2d(8)) and of the Refiner (graph/refiner.py:13,20,37,43).

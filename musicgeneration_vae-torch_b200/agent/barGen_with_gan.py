@@ -461,9 +461,10 @@ class BarGen(object):
         avg_generator_loss(loss)
         return gen_note[:3]
 
-    def generate(self, music_length=10, songs=1, seed=0):
+    def generate(self, music_length=10, songs=1, seed=0, sampler="threshold", temperature=1.0, primer=None):
         """the per-epoch sample generation of :307-328 (same loop as maker_bar.py)"""
         g = torch.Generator(device=self.device).manual_seed(seed)
         lat = torch.randn(music_length * 4, songs, 1152, device=self.device, generator=g)
         self.generator.eval()
-        return sample_songs(self.generator, lat, music_length)
+        return sample_songs(self.generator, lat, music_length, sampler=sampler, temperature=temperature,
+                            seed=g.initial_seed(), primer=primer)

@@ -286,3 +286,26 @@ def threshold_pack(probs: torch.Tensor, threshold: float, want_bits: bool = True
                                               None if out is None else out.data_ptr(), _lib.stream_ptr()),
                "threshold_pack")
     return bits, out
+
+
+def bernoulli_sample(logits: torch.Tensor, temperature: float, seed: int, song_base: int, bar_index: int,
+                     out: torch.Tensor = None) -> torch.Tensor:
+    """bvae_bernoulli_sample: draw every cell of ``logits`` (contiguous CUDA fp32, rows of 5760 cells = one bar of song
+    ``song_base + row``) as Bernoulli(sigmoid(logit / temperature)) from the counter-based stream of
+    (seed, song, bar_index, cell).  Returns {0,1} fp32 of the same shape (``out`` if given)."""
+    if not logits.is_cuda:
+        raise RuntimeError("bernoulli_sample runs on the device (libbarvae.so); there is no CPU fallback")
+    if logits.dtype != torch.float32 or not logits.is_contiguous() or logits.numel() % BAR_CELLS:
+        raise ValueError("bernoulli_sample: logits must be a contiguous fp32 tensor of whole %d-cell bars" % BAR_CELLS)
+    if not 0 <= int(seed) < 2 ** 64:
+        raise ValueError("bernoulli_sample: seed must fit in 64 unsigned bits")
+    t = float(temperature)
+    inv_t = 1.0 / t if t > 0 else float("nan")      # the library rejects a non-finite / non-positive inverse
+    if out is None:
+        out = torch.empty_like(logits)
+    elif out.dtype != torch.float32 or not out.is_contiguous() or out.numel() != logits.numel() or not out.is_cuda:
+        raise ValueError("bernoulli_sample: out must be a contiguous CUDA fp32 tensor like logits")
+    _lib.check(_lib.lib().bvae_bernoulli_sample(logits.data_ptr(), logits.numel() // BAR_CELLS, inv_t, int(seed),
+                                                int(song_base), int(bar_index), out.data_ptr(), _lib.stream_ptr()),
+               "bernoulli_sample")
+    return out

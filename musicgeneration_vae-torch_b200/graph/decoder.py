@@ -232,7 +232,22 @@ class Decoder(nn.Module):
         return _DecoderFn.apply(self, z, pre_z, phrase_feature, position, dropout_masks, *self._plist)
 
     # ---------------------------------------------------------------------------------------------------
-    def _fwd(self, z, pre_z, pf, position, masks, save):
+    def forward_logits(self, z, pre_z, phrase_feature, position):
+        """Inference only (no dropout, nothing saved for a backward pass): ``(probs, logits)``, both [B,1,96,60] fp32
+        from ONE fit2 + sigmoid launch, so ``probs`` is what ``forward`` returns and ``logits`` the values it squashed.
+        The sampling loop's Bernoulli mode draws from the logits at a temperature (data/packed.bernoulli_sample)."""
+        if torch.is_grad_enabled():
+            raise RuntimeError("Decoder.forward_logits is inference-only: call it under torch.no_grad()")
+        if self.training:
+            raise RuntimeError("Decoder.forward_logits is inference-only: put the module in eval() mode (no dropout)")
+        if not z.is_cuda:
+            raise RuntimeError("the B200 path needs CUDA tensors; there is no CPU fallback")
+        logits = torch.empty((z.shape[0], 1, 96, 60), dtype=torch.float32, device=z.device)
+        with saving(False):
+            probs, _ = self._fwd(z, pre_z, phrase_feature, position, None, False, logits=logits)
+        return probs, logits
+
+    def _fwd(self, z, pre_z, pf, position, masks, save, logits=None):
         B = z.shape[0]
         emb = self.position_embedding.weight.detach()[position]
         pcat = Act(torch.cat((pf.detach().float(), emb), 1).to(BF16), B, 1, 1, 2304)
@@ -270,7 +285,10 @@ class Decoder(nn.Module):
             h = out
         rows = B * h.H * h.W
         recon = torch.empty((B, 1, h.H, h.W), dtype=torch.float32, device=z.device)
-        _lib.check(_lib.lib().bvae_fit_sigmoid_fwd(h.ptr, h.pitch, self.fit2.weight.data_ptr(), rows, 64, None,
+        if logits is not None:
+            assert logits.dtype == torch.float32 and logits.is_contiguous() and logits.numel() == rows
+        _lib.check(_lib.lib().bvae_fit_sigmoid_fwd(h.ptr, h.pitch, self.fit2.weight.data_ptr(), rows, 64,
+                                                   None if logits is None else logits.data_ptr(),
                                                    recon.data_ptr(), _lib.stream_ptr()), "fit_sigmoid_fwd")
         saved = (position, pcat, bcat, lin, keep, x, hcat, c_p, c_t, nb, c_f, ctxs, h, recon) if save else None
         return recon, saved
