@@ -295,6 +295,23 @@ int bvae_bernoulli_sample(const float* logits /* [bars][5760] */, int64_t bars, 
                           float* out_f32 /* [bars][5760] {0,1} */, void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------
+ * Per-bar score of a given piano-roll under the decoder's Bernoulli distribution at a temperature.  For each bar,
+ * with l = logit * inv_temperature, p = 1.f / (1.f + expf(-l)) (the expression of bvae_bernoulli_sample) and t = 1 for
+ * a nonzero target cell, else 0:
+ *   nll_out[b]        = sum over the 5760 cells of (t ? softplus(-l) : softplus(l)),  softplus(x) = max(x,0) +
+ *                       log1pf(expf(-|x|))  -- in nats; the ATen equivalent is, per bar,
+ *                       binary_cross_entropy_with_logits(l, t, reduction='sum')
+ *   counts_out[b][0..2] = { #(p > threshold and t), #(p > threshold), #t }   (true positives, predicted on, target on)
+ * +-inf logits give the limits (t=1, l=+inf: 0; t=0, l=+inf: +inf); a NaN logit gives a NaN nll and is never counted
+ * as predicted on.  No atomics, fixed summation order: a bar's result depends only on its logits and target, so a call
+ * split into chunks returns the same bits as one call.  bars >= 0, inv_temperature finite and > 0, threshold finite,
+ * else BVAE_ERR_SHAPE; logits and target 16-byte aligned, nll_out and counts_out 4-byte aligned, else BVAE_ERR_ALIGN.
+ * ------------------------------------------------------------------------------------------------------------ */
+int bvae_bar_score(const float* logits /* [bars][5760] */, const float* target /* [bars][5760] {0,1} */, int64_t bars,
+                   float inv_temperature, float threshold, float* nll_out /* [bars] */,
+                   int32_t* counts_out /* [bars][3] */, void* stream);
+
+/* ------------------------------------------------------------------------------------------------------------
  * nn.BatchNorm2d(C, eps, momentum, affine) (+ optional (Leaky)ReLU) on an NHWC tensor with few channels: the norm of the
  * GAN-phase piano-roll discriminator (graph/bar_discriminator.py:19-23,69,113-114,153: BatchNorm2d(8..64, eps=1e-5,
  * momentum=0.01), OnOffFeature's default-momentum BatchNorm2d(8)) and of the Refiner (graph/refiner.py:13,20,37,43).

@@ -73,6 +73,10 @@ __device__ __forceinline__ uint4 philox4x32_10(uint4 c, uint2 k) {
   return c;
 }
 
+// The decoder's probability of a logit, with the accurate expf (no fast math).  fit_sigmoid_fwd_kernel, the Bernoulli
+// draw and the bar score all use this one expression, so at temperature 1 they agree with the decoder bit for bit.
+__device__ __forceinline__ float prob_of_logit(float l) { return 1.f / (1.f + expf(-l)); }
+
 __device__ __forceinline__ float sigmoidf_(float x) { return 1.f / (1.f + __expf(-x)); }
 __device__ __forceinline__ float act_fwd(float v, float slope) { return v > 0.f ? v : v * slope; }
 

@@ -190,7 +190,7 @@ __global__ void fit_sigmoid_fwd_kernel(const bf16* __restrict__ x, int x_pitch, 
     for (int o = G >> 1; o > 0; o >>= 1) acc += __shfl_xor_sync(0xffffffffu, acc, o);
     if (sub == 0 && row < rows) {
       if (logits) logits[row] = acc;
-      recon[row] = 1.f / (1.f + expf(-acc));
+      recon[row] = prob_of_logit(acc);
     }
   }
 }

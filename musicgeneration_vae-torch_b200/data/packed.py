@@ -309,3 +309,26 @@ def bernoulli_sample(logits: torch.Tensor, temperature: float, seed: int, song_b
                                                 int(song_base), int(bar_index), out.data_ptr(), _lib.stream_ptr()),
                "bernoulli_sample")
     return out
+
+
+def score_bars(logits: torch.Tensor, target: torch.Tensor, temperature: float = 1.0, threshold: float = 0.3):
+    """bvae_bar_score: the per-bar score of the {0,1} roll ``target`` under Bernoulli(sigmoid(logit / temperature)), the
+    distribution ``bernoulli_sample`` draws from.  Both are contiguous CUDA fp32 tensors of the same number of whole
+    5760-cell bars.  Returns ``(nll [N] fp32, counts [N, 3] int32)``: the negative log-likelihood of each bar in nats
+    (binary_cross_entropy_with_logits with reduction='sum'), and per bar the cells with p > ``threshold`` that are on in
+    the target, the cells with p > ``threshold``, and the cells on in the target."""
+    if not (logits.is_cuda and target.is_cuda):
+        raise RuntimeError("score_bars runs on the device (libbarvae.so); there is no CPU fallback")
+    for name, t in (("logits", logits), ("target", target)):
+        if t.dtype != torch.float32 or not t.is_contiguous() or t.numel() % BAR_CELLS:
+            raise ValueError("score_bars: %s must be a contiguous fp32 tensor of whole %d-cell bars" % (name, BAR_CELLS))
+    if target.numel() != logits.numel():
+        raise ValueError("score_bars: logits and target must hold the same number of bars")
+    t = float(temperature)
+    inv_t = 1.0 / t if t > 0 else float("nan")      # the library rejects a non-finite / non-positive inverse
+    bars = logits.numel() // BAR_CELLS
+    nll = torch.empty(bars, dtype=torch.float32, device=logits.device)
+    counts = torch.empty(bars, 3, dtype=torch.int32, device=logits.device)
+    _lib.check(_lib.lib().bvae_bar_score(logits.data_ptr(), target.data_ptr(), bars, inv_t, float(threshold),
+                                         nll.data_ptr(), counts.data_ptr(), _lib.stream_ptr()), "score_bars")
+    return nll, counts

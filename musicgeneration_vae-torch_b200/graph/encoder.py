@@ -61,6 +61,16 @@ class _EncoderTrunk(nn.Module):
         self._plist = list(self.parameters())
         return _TrunkFn.apply(self, x, *self._plist)
 
+    def encode(self, x):
+        """Inference only: ``forward(x)`` without the autograd node and with nothing saved for a backward pass (under
+        ``torch.no_grad`` the node would still save, because the parameters require grad).  ``x`` may be fp32 or bf16."""
+        if torch.is_grad_enabled():
+            raise RuntimeError("encode is inference-only: call it under torch.no_grad()")
+        if not x.is_cuda:
+            raise RuntimeError("the B200 path needs CUDA tensors; there is no CPU fallback")
+        with saving(False):
+            return self._fwd(x, False)[0]
+
     # ---- fused forward / backward over engine.Act views ------------------------------------------------
     def _fwd(self, x, save):
         B, _, H, W = x.shape
