@@ -60,9 +60,8 @@ const char* bvae_last_kernel(void);
  * reductions stay atomic (DESIGN.md section 7). */
 void bvae_set_deterministic(int on);
 int bvae_deterministic(void);
-/* Kernel-variant switches kept for A/B measurements (DESIGN.md section 4): BVAE_CONV_V1, BVAE_CONV_TMA_STORE, BVAE_CONV_HALO,
- * BVAE_WGRAD_HALO, BVAE_WGRAD_MC, BVAE_WGRAD_SPLITS, BVAE_WGRAD_WIDE_TMA, BVAE_WGRAD_STAGES, BVAE_NB_MLP, BVAE_NB_MODE, BVAE_NB_SPLIT, BVAE_NB_FAST, BVAE_NB_SMALL (+ its thresholds
- * BVAE_NB_SMALL_HW / BVAE_NB_SMALL_N).  Each is read per call as: the value set here,
+/* Norm-block kernel-variant switches kept for A/B measurements (DESIGN.md section 4.3): BVAE_NB_MLP, BVAE_NB_MODE, BVAE_NB_SPLIT,
+ * BVAE_NB_FAST, BVAE_NB_SMALL (+ its thresholds BVAE_NB_SMALL_HW / BVAE_NB_SMALL_N).  Each is read per call as: the value set here,
  * else the environment variable of the same name, else its default; value < 0 removes the override.  Every variant is
  * parity-tested (tests/test_gpu_kernels.py::test_kernel_variants_*). */
 void bvae_set_option(const char* name, int value);

@@ -34,13 +34,11 @@ static bvae_conv_desc single_phase(const bvae_conv_desc* d, int i) {
   return s;
 }
 
-namespace bvae { int conv_tc_multi_ok(const bvae_conv_desc* d); }
-
 extern "C" int bvae_conv_gemm(const bvae_conv_desc* d, int impl, void* stream) {
   BVAE_REQUIRE(d && d->x && d->w && d->y, BVAE_ERR_SHAPE, "conv_gemm: null pointer");
   if (d->nphase > 0) {
     BVAE_REQUIRE(d->nphase <= BVAE_MAX_PHASES, BVAE_ERR_SHAPE, "conv_gemm: nphase=%d", d->nphase);
-    if (!(impl != BVAE_IMPL_SIMT && conv_tc_multi_ok(d))) {
+    if (!(impl != BVAE_IMPL_SIMT && conv_tc_eligible(d))) {
       for (int i = 0; i < d->nphase; ++i) {          // kernels that take one phase at a time
         if (d->ph_QH[i] <= 0 || d->ph_QW[i] <= 0) continue;
         const bvae_conv_desc s = single_phase(d, i);
@@ -84,7 +82,7 @@ extern "C" int bvae_conv_gemm(const bvae_conv_desc* d, int impl, void* stream) {
 extern "C" int bvae_conv_stats_ok(const bvae_conv_desc* d) {
   if (!d) return 0;
   if (d->nphase > 0) {
-    if (conv_tc_multi_ok(d)) return conv_tc_stats_ok(d);
+    if (conv_tc_eligible(d)) return conv_tc_stats_ok(d);
     for (int i = 0; i < d->nphase; ++i) {
       if (d->ph_QH[i] <= 0 || d->ph_QW[i] <= 0) continue;
       const bvae_conv_desc s = single_phase(d, i);

@@ -1,6 +1,6 @@
 // conv_tc.cu -- tcgen05 / TMEM / TMA implicit-GEMM kernels for sm_100a.
 //
-// conv_tc_kernel  (forward + data gradient, operands K-major):
+// conv_tc2_kernel (forward + data gradient, operands K-major):
 //   D[128 pixels x BN channels] (fp32, TMEM) = sum over (tap, channel block) A[128 x KB] * B[BN x KB]^T
 //   A = activation patch: ONE tiled TMA box {KB channels, bw, bh, bn} of an NHWC view per (tap, channel block);
 //       the tap shift is a coordinate offset, padding is TMA out-of-bounds zero fill, a strided (stride-2 / k==s)
@@ -155,24 +155,6 @@ __device__ __forceinline__ void umma_f16_steps(uint32_t tmem_d, uint64_t adesc, 
 __device__ __forceinline__ void umma_commit(uint64_t* bar) {
   asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.b64 [%0];" ::"r"(smem_u32(bar)) : "memory");
 }
-// ---- 2-CTA cluster helpers (wgrad_tc_kernel with TMA multicast of the shared operand)
-__device__ __forceinline__ void cluster_sync_all() {
-  asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// the box lands at the same shared-memory offset of every CTA in `mask`, and each of them gets the complete_tx on its own
-// barrier at the same offset
-__device__ __forceinline__ void tma_load_4d_mc(void* dst, const CUtensorMap* map, uint64_t* bar, int c0, int c1, int c2,
-                                               int c3, uint16_t mask) {
-  asm volatile(
-      "cp.async.bulk.tensor.4d.shared::cluster.global.mbarrier::complete_tx::bytes.multicast::cluster"
-      " [%0], [%1, {%3, %4, %5, %6}], [%2], %7;"
-      ::"r"(smem_u32(dst)), "l"((uint64_t)map), "r"(smem_u32(bar)), "r"(c0), "r"(c1), "r"(c2), "r"(c3), "h"(mask) : "memory");
-}
-// like umma_commit, arriving on the barrier at this offset in every CTA of `mask`
-__device__ __forceinline__ void umma_commit_mc(uint64_t* bar, uint16_t mask) {
-  asm volatile("tcgen05.commit.cta_group::1.mbarrier::arrive::one.shared::cluster.multicast::cluster.b64 [%0], %1;"
-               ::"r"(smem_u32(bar)), "h"(mask) : "memory");
-}
 // 32 lanes x 32 consecutive fp32 columns -> 32 registers per thread
 __device__ __forceinline__ void tmem_ld32(uint32_t taddr, uint32_t* v) {
   asm volatile(
@@ -213,7 +195,7 @@ struct alignas(64) ConvTcParams {
   int ntaps, kchunks, C;
   int bw, bh, bn, tiles_w, tiles_h, tiles_n, n_tiles;
   int N, QH, QW, Cout;
-  int nphase;                                   // >= 1 (conv_tc2 only; conv_tc_kernel handles exactly one phase)
+  int nphase;                                   // >= 1
   int ph_tap0[BVAE_MAX_PHASES], ph_ntaps[BVAE_MAX_PHASES], ph_ooy[BVAE_MAX_PHASES], ph_oox[BVAE_MAX_PHASES];
   int ph_QH[BVAE_MAX_PHASES], ph_QW[BVAE_MAX_PHASES];
   void* y;
@@ -225,7 +207,7 @@ struct alignas(64) ConvTcParams {
   float slope, mask_slope;
   // halo mode (stride-1 multi-tap layers with resident weights): ONE activation tile with its halo is loaded per
   // (output tile, K chunk) and every tap reads it through a row-shifted shared-memory descriptor
-  // TMA-store epilogue (BN <= 128): one output tensor map per phase, box {32 floats or 64 bf16, bw, bh, bn}
+  // TMA-store epilogue (fp32 outputs, BN <= 128): one output tensor map per phase, box {32 floats, bw, bh, bn}
   CUtensorMap ymap[BVAE_MAX_PHASES];
   int tma_store;
   int halo, halo_x0, halo_y0, halo_rows, halo_stage, halo_stages;
@@ -251,154 +233,10 @@ __device__ __forceinline__ float warp_col_reduce(float (&v)[32], Op op) {
 }
 
 // ---------------------------------------------------------------------------------------------------------
-// forward / dgrad kernel.  128 threads: warp 0 = TMA producer, warp 1 = MMA issuer, warp 2 = TMEM allocator,
-// then all four warps run the epilogue (warp w owns TMEM lanes 32w..32w+31 = tile rows).
-// ---------------------------------------------------------------------------------------------------------
-template <int KB, int BN, int STAGES>
-__global__ void __launch_bounds__(128) conv_tc_kernel(const __grid_constant__ ConvTcParams p) {
-  constexpr int A_BYTES = 128 * KB * 2;
-  constexpr int B_BYTES = BN * KB * 2;
-  constexpr int STAGE_BYTES = A_BYTES + B_BYTES;
-  constexpr int TMEM_COLS = BN <= 32 ? 32 : (BN <= 64 ? 64 : (BN <= 128 ? 128 : 256));
-  constexpr uint32_t LAYOUT = KB == 64 ? 2u : 4u;           // SWIZZLE_128B : SWIZZLE_64B
-  constexpr uint32_t SBO = 8 * KB * 2;                      // 8 rows of KB bf16
-  constexpr uint32_t IDESC = make_idesc(128, BN, 0, 0);
-
-  extern __shared__ uint8_t smem_raw[];
-  uint8_t* smem = (uint8_t*)(((uintptr_t)smem_raw + 1023) & ~(uintptr_t)1023);
-  uint64_t* full_bar = (uint64_t*)(smem + STAGES * STAGE_BYTES);
-  uint64_t* empty_bar = full_bar + STAGES;
-  uint64_t* tmem_full = empty_bar + STAGES;
-  uint32_t* tmem_slot = (uint32_t*)(tmem_full + 1);
-  float* s_bias = (float*)(tmem_slot + 2);
-
-  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const int n_tile = blockIdx.x % p.n_tiles;
-  int m_tile = blockIdx.x / p.n_tiles;
-  const int tw = m_tile % p.tiles_w; m_tile /= p.tiles_w;
-  const int th = m_tile % p.tiles_h;
-  const int tn = m_tile / p.tiles_h;
-  const int KT = p.ntaps * p.kchunks;
-
-  if (warp == 0 && lane == 0) {
-    for (int s = 0; s < STAGES; ++s) { mbar_init(full_bar + s, 1); mbar_init(empty_bar + s, 1); }
-    mbar_init(tmem_full, 1);
-    fence_barrier_init();
-    tma_prefetch_desc(&p.bmap);
-    tma_prefetch_desc(&p.amap[0]);
-  }
-  if (warp == 2) tmem_alloc<TMEM_COLS>(tmem_slot);
-  for (int i = threadIdx.x; i < BN; i += 128) s_bias[i] = p.bias ? p.bias[n_tile * BN + i] : 0.f;
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-
-  if (warp == 0 && lane == 0) {
-    // ---------------- TMA producer ----------------
-    const uint32_t tx = (uint32_t)(p.bn * p.bh * p.bw * KB * 2 + B_BYTES);
-    int kb = 0;
-    for (int t = 0; t < p.ntaps; ++t) {
-      const CUtensorMap* am = &p.amap[p.tap_view[t]];
-      const int cw = tw * p.bw + p.tap_ex[t], ch = th * p.bh + p.tap_ey[t], cn = tn * p.bn;
-      for (int kc = 0; kc < p.kchunks; ++kc, ++kb) {
-        const int s = kb % STAGES;
-        const uint32_t ph = (uint32_t)(kb / STAGES) & 1u;
-        mbar_wait(empty_bar + s, ph ^ 1u);
-        mbar_expect_tx(full_bar + s, tx);
-        uint8_t* sa = smem + s * STAGE_BYTES;
-        tma_load_4d(sa, am, full_bar + s, kc * KB, cw, ch, cn);
-        tma_load_2d(sa + A_BYTES, &p.bmap, full_bar + s, t * p.C + kc * KB, n_tile * BN);
-      }
-    }
-  } else if (warp == 1 && lane == 0) {
-    // ---------------- MMA issuer ----------------
-    for (int kb = 0; kb < KT; ++kb) {
-      const int s = kb % STAGES;
-      const uint32_t ph = (uint32_t)(kb / STAGES) & 1u;
-      mbar_wait(full_bar + s, ph);
-      tc_fence_after();
-      const uint32_t sa = smem_u32(smem + s * STAGE_BYTES);
-      const uint64_t adesc = make_sdesc(sa, 16, SBO, LAYOUT);
-      const uint64_t bdesc = make_sdesc(sa + A_BYTES, 16, SBO, LAYOUT);
-#pragma unroll
-      for (int j = 0; j < KB / 16; ++j)      // +32 bytes (= 2 in the >>4 encoded start address) per K=16 step
-        umma_f16(tmem_base, adesc + 2 * j, bdesc + 2 * j, IDESC, (kb | j) ? 1u : 0u);
-      umma_commit(empty_bar + s);            // frees the smem slot when these MMAs retire
-    }
-    umma_commit(tmem_full);
-  }
-  __syncwarp();
-  mbar_wait(tmem_full, 0);
-  tc_fence_after();
-
-  // ---------------- epilogue: TMEM -> registers -> global ----------------
-  const int r = threadIdx.x;
-  const int rows_box = p.bn * p.bh * p.bw;
-  const int nn = r / (p.bh * p.bw), hh = (r / p.bw) % p.bh, ww = r % p.bw;
-  const int n = tn * p.bn + nn, qy = th * p.bh + hh, qx = tw * p.bw + ww;
-  const bool valid = r < rows_box && n < p.N && qy < p.QH && qx < p.QW;
-  const int64_t opix = ((int64_t)n * p.OH + (qy * p.osy + p.ooy)) * p.OW + (qx * p.osx + p.oox);
-  const int col0 = n_tile * BN;
-#pragma unroll 1
-  for (int c0 = 0; c0 < BN; c0 += 32) {
-    uint32_t v[32];
-    tmem_ld32(tmem_base + ((uint32_t)(warp * 32) << 16) + (uint32_t)c0, v);
-    if (!valid) continue;
-    float f[32];
-#pragma unroll
-    for (int i = 0; i < 32; ++i) {
-      f[i] = __uint_as_float(v[i]) + s_bias[c0 + i];
-      if (p.act) f[i] = act_fwd(f[i], p.slope);
-    }
-    if (p.addend) {
-      if (p.out_f32) {
-        const float* ap = (const float*)p.addend + opix * p.add_pitch + col0 + c0;
-#pragma unroll
-        for (int i = 0; i < 32; i += 4) {
-          const float4 a = *reinterpret_cast<const float4*>(ap + i);
-          f[i] += a.x; f[i + 1] += a.y; f[i + 2] += a.z; f[i + 3] += a.w;
-        }
-      } else {
-        const bf16* ap = (const bf16*)p.addend + opix * p.add_pitch + col0 + c0;
-#pragma unroll
-        for (int i = 0; i < 32; i += 8) {
-          float a[8];
-          unpack8(ldg8(ap + i), a);
-#pragma unroll
-          for (int k = 0; k < 8; ++k) f[i + k] += a[k];
-        }
-      }
-    }
-    if (p.mask) {
-      const bf16* mp = (const bf16*)p.mask + opix * p.mask_pitch + col0 + c0;
-#pragma unroll
-      for (int i = 0; i < 32; i += 8) {
-        float a[8];
-        unpack8(ldg8(mp + i), a);
-#pragma unroll
-        for (int k = 0; k < 8; ++k) f[i + k] *= (a[k] > 0.f) ? 1.f : p.mask_slope;
-      }
-    }
-    if (p.out_f32) {
-      float* yp = (float*)p.y + opix * p.y_pitch + col0 + c0;
-#pragma unroll
-      for (int i = 0; i < 32; i += 4) *reinterpret_cast<float4*>(yp + i) = make_float4(f[i], f[i + 1], f[i + 2], f[i + 3]);
-    } else {
-      bf16* yp = (bf16*)p.y + opix * p.y_pitch + col0 + c0;
-#pragma unroll
-      for (int i = 0; i < 32; i += 8) stg8(yp + i, pack8(f + i));
-    }
-  }
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 2) tmem_dealloc<TMEM_COLS>(tmem_base);
-}
-
-// ---------------------------------------------------------------------------------------------------------
-// persistent variant: one CTA per SM loops over output tiles.  256 threads: warp 0 = TMA producer, warp 1 = MMA
-// issuer, warp 2 = TMEM allocator, warps 4..7 = epilogue.  Two TMEM accumulator buffers (2 x BN columns) let the
-// epilogue of tile i overlap the main loop of tile i+1; barrier init / TMEM allocation are paid once per CTA.
+// forward / data-gradient kernel, persistent: one CTA per SM loops over output tiles.  256 threads: warp 0 = TMA
+// producer, warp 1 = MMA issuer, warp 2 = TMEM allocator, warps 4..7 = epilogue.  Two TMEM accumulator buffers (2 x BN
+// columns) let the epilogue of tile i overlap the main loop of tile i+1; barrier init / TMEM allocation are paid once per
+// CTA.
 // ---------------------------------------------------------------------------------------------------------
 __device__ __forceinline__ void mbar_arrive(uint64_t* bar) {
   asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
@@ -602,17 +440,15 @@ __global__ void __launch_bounds__(ConvTc2Cfg<BN>::THREADS, 1) conv_tc2_kernel(co
       tc_fence_after();
       const uint32_t tacc = tmem_base + ab * ACC_COLS + ((uint32_t)(wq * 32) << 16);
       if (BN <= 128 && p.tma_store) {
-        // Output through shared memory and one tiled TMA store per 128-byte-wide slab (32 fp32 / 64 bf16 columns):
-        // the direct path issues, per warp instruction, 32 separate 16-byte requests to 32 different rows (2048 L1
-        // requests per 128x64 fp32 tile), which made the epilogue the longest stage of the small-K layers.  Rows and
-        // columns outside the output are clipped by the store.
-        const int CS = p.out_f32 ? 32 : 64;                 // columns per slab
+        // fp32 output through shared memory and one tiled TMA store per 128-byte-wide slab (32 columns): the direct
+        // path issues, per warp instruction, 32 separate 16-byte requests to 32 different rows (2048 L1 requests per
+        // 128x64 fp32 tile), which made the epilogue the longest stage of the small-K layers.  Rows and columns outside
+        // the output are clipped by the store.
 #pragma unroll(PRE ? 2 : 1)
         for (int c0 = 0; c0 < BN; c0 += 32) {
           uint32_t v[32];
           tmem_ld32(tacc + (uint32_t)c0, v);
           if (c0 + 32 >= BN) { tc_fence_before(); mbar_arrive(tempty + ab); }     // accumulator drained
-          const int cs0 = c0 & ~(CS - 1);                   // first column of this slab
           uint8_t* slab = yslabs + (gsl & 1u) * 16384u;
           float f[32];
 #pragma unroll
@@ -629,22 +465,11 @@ __global__ void __launch_bounds__(ConvTc2Cfg<BN>::THREADS, 1) conv_tc2_kernel(co
             for (int i = 0; i < 32; ++i) f[i] = act_fwd(f[i], p.slope);
           }
           if (p.addend && valid) {
-            if (p.out_f32) {
-              const float* ap = (const float*)p.addend + opix * p.add_pitch + col0 + c0;
+            const float* ap = (const float*)p.addend + opix * p.add_pitch + col0 + c0;
 #pragma unroll
-              for (int i = 0; i < 32; i += 4) {
-                const float4 a = *reinterpret_cast<const float4*>(ap + i);
-                f[i] += a.x; f[i + 1] += a.y; f[i + 2] += a.z; f[i + 3] += a.w;
-              }
-            } else {
-              const bf16* ap = (const bf16*)p.addend + opix * p.add_pitch + col0 + c0;
-#pragma unroll
-              for (int i = 0; i < 32; i += 8) {
-                float a[8];
-                unpack8((PRE && pre_add) ? pre_a[PRE ? ((c0 + i) / 8) % NPRE : 0] : ldg8(ap + i), a);
-#pragma unroll
-                for (int k = 0; k < 8; ++k) f[i + k] += a[k];
-              }
+            for (int i = 0; i < 32; i += 4) {
+              const float4 a = *reinterpret_cast<const float4*>(ap + i);
+              f[i] += a.x; f[i + 1] += a.y; f[i + 2] += a.z; f[i + 3] += a.w;
             }
           }
           if (p.mask && valid) {
@@ -659,28 +484,16 @@ __global__ void __launch_bounds__(ConvTc2Cfg<BN>::THREADS, 1) conv_tc2_kernel(co
           }
           uint8_t* row = slab + r * 128;
           const int sw = r & 7;
-          if (p.out_f32) {
-            // the store issued from this slab buffer two slabs ago must have finished reading it
-            if (r == 0) tma_store_wait_read<1>();
-            epi_bar_sync(eg);
+          // the store issued from this slab buffer two slabs ago must have finished reading it
+          if (r == 0) tma_store_wait_read<1>();
+          epi_bar_sync(eg);
 #pragma unroll
-            for (int j = 0; j < 8; ++j)
-              *reinterpret_cast<float4*>(row + ((j ^ sw) << 4)) = make_float4(f[4 * j], f[4 * j + 1], f[4 * j + 2], f[4 * j + 3]);
-          } else {
-            const int half = (c0 - cs0) >> 5;               // which 64-byte half of the 128-byte row
-            if (half == 0) {
-              if (r == 0) tma_store_wait_read<1>();
-              epi_bar_sync(eg);
-            }
-#pragma unroll
-            for (int j = 0; j < 4; ++j)
-              *reinterpret_cast<uint4*>(row + (((4 * half + j) ^ sw) << 4)) = pack8(f + 8 * j);
-            if (half == 0) continue;                        // the slab is complete after its second half
-          }
+          for (int j = 0; j < 8; ++j)
+            *reinterpret_cast<float4*>(row + ((j ^ sw) << 4)) = make_float4(f[4 * j], f[4 * j + 1], f[4 * j + 2], f[4 * j + 3]);
           fence_proxy_async();
           epi_bar_sync(eg);
           if (r == 0) {
-            tma_store_4d(&p.ymap[ph], slab, col0 + cs0, tw * p.bw, th * p.bh, tn * p.bn);
+            tma_store_4d(&p.ymap[ph], slab, col0 + c0, tw * p.bw, th * p.bh, tn * p.bn);
             tma_store_commit();
           }
           ++gsl;
@@ -809,7 +622,6 @@ struct alignas(64) WgradTcParams {
   int bw, bh, bn, chunks_w, chunks_h, chunks_n, nchunks, chunks_per_split, splits;
   int a_atoms;                      // 64-channel atoms of the anchor tile actually loaded (1 or 2)
   int ra_tiles, rs_tiles;
-  int mc;                           // 2: launched as 2-CTA clusters that share the shifted tile (TMA multicast); else 1
   int wt;                           // 1: "wide TMA" -- amap / smap are 5-D {64 ch, W, H, N, channel block} maps, one request per operand
   int wt_stages, wt_stage_bytes;    // WT: ring depth (2..4) and bytes per stage = atoms * rows_box * 128 (packed atoms)
   int Ca, Cs;
@@ -830,7 +642,7 @@ struct alignas(64) WgradTcParams {
 // C/64} a box {64, bw, bh, bn, atoms} lands as `atoms` consecutive [rows][64 ch] swizzled tiles: ONE request per operand and
 // tap (3 per stage instead of 10).  The tiles are packed (rows_box * 128 B apart, the descriptors' leading-dimension offset),
 // every row of every tile is rewritten by each request (out-of-bounds pixels arrive as zeros), so the ring needs no zeroing.
-template <int CB, int NS, int STAGES, bool MC = false, bool WT = false>
+template <int CB, int NS, int STAGES, bool WT = false>
 __global__ void __launch_bounds__(128) wgrad_tc_kernel(const __grid_constant__ WgradTcParams p) {
   constexpr int KP = 64;
   constexpr int ROW_BYTES = CB * 2;
@@ -858,19 +670,11 @@ __global__ void __launch_bounds__(128) wgrad_tc_kernel(const __grid_constant__ W
   uint32_t* tmem_slot = (uint32_t*)(tmem_full + 1);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  // mc == 2: CTAs 2k and 2k+1 form a cluster.  They own the anchor tiles 2j and 2j+1 of the SAME (shifted tile, tap group,
-  // pixel split), so every shifted atom is needed by both: each CTA fetches every other atom and multicasts it into both
-  // shared memories (L2 -> SM bytes per 64-pixel chunk: 16 KB + 32 KB instead of 16 KB + 64 KB for NS = 256, the traffic
-  // that bounds these layers at half of the tensor peak).  A stage may be refilled only when BOTH CTAs have consumed
-  // it, so the MMA commits arrive on the empty barrier of both (count 2).
-  constexpr bool mc = MC;             // a template parameter: the runtime flag cost the default kernels 5-15 % (producer issue path)
   int b = blockIdx.x;
-  const int rank = mc ? (b & 1) : 0;
-  if (mc) b >>= 1;
   const int split = b % p.splits; b /= p.splits;
   const int tg = b % p.tap_groups; b /= p.tap_groups;
   const int rs_tile = b % p.rs_tiles;
-  const int ra_tile = mc ? (b / p.rs_tiles) * 2 + rank : b / p.rs_tiles;
+  const int ra_tile = b / p.rs_tiles;
   const int tap0 = tg * p.tpc;
   const int ntap = min(p.tpc, p.ntaps - tap0);
   const int ck0 = split * p.chunks_per_split;
@@ -884,7 +688,7 @@ __global__ void __launch_bounds__(128) wgrad_tc_kernel(const __grid_constant__ W
   }
   const uint32_t atom_stride = WT ? (uint32_t)(rows_box * ROW_BYTES) : (uint32_t)ATOM_BYTES;   // distance between channel atoms
   if (warp == 0 && lane == 0) {
-    for (int s = 0; s < MAXST; ++s) { mbar_init(full_bar + s, 1); mbar_init(empty_bar + s, mc ? 2 : 1); }
+    for (int s = 0; s < MAXST; ++s) { mbar_init(full_bar + s, 1); mbar_init(empty_bar + s, 1); }
     mbar_init(tmem_full, 1);
     fence_barrier_init();
     tma_prefetch_desc(&p.amap);
@@ -893,11 +697,10 @@ __global__ void __launch_bounds__(128) wgrad_tc_kernel(const __grid_constant__ W
   tc_fence_before();
   __syncthreads();
   tc_fence_after();
-  if (mc) cluster_sync_all();        // the peer's barriers are initialised and its buffer zeroed before anything is multicast
   const uint32_t tmem_base = *tmem_slot;
 
   if (warp == 0 && lane == 0) {
-    const uint32_t tx = (uint32_t)(rows_box * ROW_BYTES * (p.a_atoms + ntap * S_ATOMS));   // bytes landing HERE (own + peer's loads)
+    const uint32_t tx = (uint32_t)(rows_box * ROW_BYTES * (p.a_atoms + ntap * S_ATOMS));
     int s = 0;
     uint32_t ph = 0;
     for (int ck = ck0; ck < ck1; ++ck) {
@@ -921,14 +724,9 @@ __global__ void __launch_bounds__(128) wgrad_tc_kernel(const __grid_constant__ W
       for (int t = 0; !WT && t < ntap; ++t) {
         const int tap = tap0 + t;
         const CUtensorMap* sm = &p.smap[p.tap_view[tap]];
-        for (int a = 0; a < S_ATOMS; ++a) {
-          if (!mc)
-            tma_load_4d(st + (A_ATOMS + t * S_ATOMS + a) * ATOM_BYTES, sm, full_bar + s, rs_tile * NS + a * CB,
-                        cw + p.tap_ex[tap], ch + p.tap_ey[tap], cn);
-          else if (((t * S_ATOMS + a) & 1) == rank)
-            tma_load_4d_mc(st + (A_ATOMS + t * S_ATOMS + a) * ATOM_BYTES, sm, full_bar + s, rs_tile * NS + a * CB,
-                           cw + p.tap_ex[tap], ch + p.tap_ey[tap], cn, (uint16_t)3);
-        }
+        for (int a = 0; a < S_ATOMS; ++a)
+          tma_load_4d(st + (A_ATOMS + t * S_ATOMS + a) * ATOM_BYTES, sm, full_bar + s, rs_tile * NS + a * CB,
+                      cw + p.tap_ex[tap], ch + p.tap_ey[tap], cn);
       }
       if (++s == nst) { s = 0; ph ^= 1u; }
     }
@@ -958,8 +756,7 @@ __global__ void __launch_bounds__(128) wgrad_tc_kernel(const __grid_constant__ W
               umma_f16(tmem_base + (uint32_t)(t * NS), adesc + KSTEP * j, bdesc + KSTEP * j, idesc, (it | j) ? 1u : 0u);
           }
         }
-        if (mc) umma_commit_mc(empty_bar + s, (uint16_t)3);
-        else umma_commit(empty_bar + s);
+        umma_commit(empty_bar + s);
       }
       __syncwarp();
       if (++s == nst) { s = 0; ph ^= 1u; }
@@ -996,7 +793,6 @@ __global__ void __launch_bounds__(128) wgrad_tc_kernel(const __grid_constant__ W
   }
   tc_fence_before();
   __syncthreads();
-  if (mc) cluster_sync_all();        // no CTA leaves while its peer may still arrive on its barriers
   if (warp == 2) tmem_dealloc<512>(tmem_base);
 }
 
@@ -1230,17 +1026,16 @@ static int make_view_map5(CUtensorMap* m, const void* base, int C, int Wv, int H
   return BVAE_OK;
 }
 
-// output view {C, Wv, Hv, N} (strides in elements), box {128 B of channels (32 floats / 64 bf16), bw, bh, bn}, 128B swizzle
-static int make_out_map(CUtensorMap* m, const void* base, bool f32, int C, int Wv, int Hv, int N, int64_t sw_elems,
-                        int64_t sh_elems, int64_t sn_elems, int bw, int bh, int bn) {
+// fp32 output view {C, Wv, Hv, N} (strides in elements), box {32 floats = 128 B of channels, bw, bh, bn}, 128B swizzle
+static int make_out_map(CUtensorMap* m, const float* base, int C, int Wv, int Hv, int N, int64_t sw_elems, int64_t sh_elems,
+                        int64_t sn_elems, int bw, int bh, int bn) {
   EncodeTiledFn enc = get_encode();
   BVAE_REQUIRE(enc, BVAE_ERR_CUDA, "cuTensorMapEncodeTiled is not available from the driver");
-  const cuuint64_t es_ = f32 ? 4 : 2;
   cuuint64_t dims[4] = {(cuuint64_t)C, (cuuint64_t)Wv, (cuuint64_t)Hv, (cuuint64_t)N};
-  cuuint64_t strides[3] = {(cuuint64_t)sw_elems * es_, (cuuint64_t)sh_elems * es_, (cuuint64_t)sn_elems * es_};
-  cuuint32_t box[4] = {f32 ? 32u : 64u, (cuuint32_t)bw, (cuuint32_t)bh, (cuuint32_t)bn};
+  cuuint64_t strides[3] = {(cuuint64_t)sw_elems * 4, (cuuint64_t)sh_elems * 4, (cuuint64_t)sn_elems * 4};
+  cuuint32_t box[4] = {32, (cuuint32_t)bw, (cuuint32_t)bh, (cuuint32_t)bn};
   cuuint32_t es[4] = {1, 1, 1, 1};
-  CUresult r = enc(m, f32 ? CU_TENSOR_MAP_DATA_TYPE_FLOAT32 : CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<void*>(base), dims, strides, box, es,
+  CUresult r = enc(m, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 4, const_cast<float*>(base), dims, strides, box, es,
                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_NONE,
                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   BVAE_REQUIRE(r == CUDA_SUCCESS, BVAE_ERR_CUDA, "cuTensorMapEncodeTiled(out) failed: %d (dims %d,%d,%d,%d box %d,%d,%d)",
@@ -1261,10 +1056,6 @@ static int make_w_map(CUtensorMap* m, const void* base, int K, int rows, int pit
   BVAE_REQUIRE(r == CUDA_SUCCESS, BVAE_ERR_CUDA, "cuTensorMapEncodeTiled(2d) failed: %d (K %d rows %d pitch %d box %d,%d)",
                (int)r, K, rows, pitch, box_k, box_rows);
   return BVAE_OK;
-}
-
-static bool use_conv_v1_flag() {
-  return option("BVAE_CONV_V1", 0) == 1;
 }
 
 static inline int floordiv(int a, int b) { return (a >= 0) ? a / b : -((-a + b - 1) / b); }
@@ -1362,10 +1153,8 @@ int conv_tc_eligible(const bvae_conv_desc* d) {
   return pick_bn(d->Cout) != 0;
 }
 
-int conv_tc_multi_ok(const bvae_conv_desc* d) { return !use_conv_v1_flag() && conv_tc_eligible(d); }
-
 int conv_tc_stats_ok(const bvae_conv_desc* d) {
-  if (use_conv_v1_flag() || !conv_tc_eligible(d) || !d->out_f32 || d->act || d->addend || d->mask) return 0;
+  if (!conv_tc_eligible(d) || !d->out_f32 || d->act || d->addend || d->mask) return 0;
   int QHm = d->QH, QWm = d->QW;
   for (int i = 0; i < d->nphase; ++i) {
     if (i == 0) QHm = QWm = 0;
@@ -1375,20 +1164,6 @@ int conv_tc_stats_ok(const bvae_conv_desc* d) {
   int bw, bh, bn;
   pick_box(d->N, QHm, QWm, 128, &bw, &bh, &bn);
   return bn == 1;
-}
-
-template <int KB, int BN, int STAGES>
-static int launch_conv(const ConvTcParams& P, int grid, cudaStream_t stream) {
-  constexpr int smem = 1024 + STAGES * (128 * KB * 2 + BN * KB * 2) + (2 * STAGES + 1) * 8 + 8 + BN * 4;
-  static bool attr_done = false;
-  if (!attr_done) {
-    cudaError_t e = cudaFuncSetAttribute(conv_tc_kernel<KB, BN, STAGES>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-    BVAE_REQUIRE(e == cudaSuccess, BVAE_ERR_CUDA, "conv_tc: cudaFuncSetAttribute(%d) failed: %s", smem, cudaGetErrorString(e));
-    attr_done = true;
-  }
-  conv_tc_kernel<KB, BN, STAGES><<<grid, 128, smem, stream>>>(P);
-  note_kernel("conv_tc_kernel<%d,%d,%d>", KB, BN, STAGES);
-  return check_launch("conv_tc");
 }
 
 template <int KB, int BN, bool BRES>
@@ -1425,24 +1200,11 @@ static int launch_conv2(const ConvTcParams& P, long tiles, cudaStream_t stream) 
   return bres ? launch_conv2_impl<KB, BN, true>(P, tiles, stream) : launch_conv2_impl<KB, BN, false>(P, tiles, stream);
 }
 
-// BVAE_CONV_TMA_STORE: 0 = direct-store epilogue everywhere, 1 (default) = TMA store for fp32 outputs, 2 = also for bf16
-// outputs (measured slower on the masked data gradients: 0.79 vs 0.65 ms on 64->64 3x3, the mask rows are already
-// prefetched there and the extra barriers cost more than the store requests save)
-static int conv_tma_store_mode() {
-  return option("BVAE_CONV_TMA_STORE", 1);
-}
-
-// BVAE_CONV_HALO: 0 = off, 1 = on (default)
-static int conv_halo_mode() {
-  return option("BVAE_CONV_HALO", 1);
-}
-
 // Halo mode applies to single-phase stride-1 layers whose weights stay resident (see launch_conv2): the output tile is
 // RH image rows of the PADDED width PW = QW + (dx_max - dx_min), flattened, so that tap (dy, dx) is the same smem tile
 // shifted by (dy - dy_min) * PW + (dx - dx_min) rows.  Output rows that fall on padding columns are discarded.
 static int plan_halo(const bvae_conv_desc* d, ConvTcParams* P, int KB, int BN) {
-  const int mode = conv_halo_mode();
-  if (mode == 0 || use_conv_v1_flag() || KB != 64 || P->nphase != 1 || d->sy != 1 || d->sx != 1 || d->osy != 1 || d->osx != 1 ||
+  if (KB != 64 || P->nphase != 1 || d->sy != 1 || d->sx != 1 || d->osy != 1 || d->osx != 1 ||
       P->n_tiles != 1 || d->ntaps < 4 || d->stats)
     return BVAE_OK;
   if ((long)d->ntaps * P->kchunks * (BN * KB * 2) > 72 * 1024) return BVAE_OK;
@@ -1472,10 +1234,6 @@ static int plan_halo(const bvae_conv_desc* d, ConvTcParams* P, int KB, int BN) {
   P->bw = PW; P->bh = RH; P->bn = 1;
   P->tiles_w = 1; P->tiles_h = ceil_div(QH, RH); P->tiles_n = d->N;
   return BVAE_OK;
-}
-
-static bool use_conv_v1() {
-  return option("BVAE_CONV_V1", 0) == 1;
 }
 
 int conv_tc_launch(const bvae_conv_desc* d, cudaStream_t stream) {
@@ -1526,14 +1284,12 @@ int conv_tc_launch(const bvae_conv_desc* d, cudaStream_t stream) {
   P.slope = d->slope; P.mask_slope = d->mask_slope;
   rc = plan_halo(d, &P, KB, BN);
   if (rc) return rc;
-  const bool f32o = d->out_f32 != 0;
-  if (conv_tma_store_mode() != 0 && (f32o || conv_tma_store_mode() == 2) && !use_conv_v1() && !d->stats && BN <= 128 &&
-      (f32o || BN >= 64) &&
-      d->y_pitch % (f32o ? 4 : 8) == 0 && ((uintptr_t)d->y & 15) == 0) {
+  // TMA-store epilogue for fp32 outputs only: on the bf16 data gradients it measured slower (0.79 vs 0.65 ms on 64->64 3x3,
+  // the mask rows are already prefetched there and the extra barriers cost more than the store requests save)
+  if (d->out_f32 && !d->stats && BN <= 128 && d->y_pitch % 4 == 0 && ((uintptr_t)d->y & 15) == 0) {
     for (int i = 0; i < P.nphase; ++i) {
-      const int64_t off = ((int64_t)P.ph_ooy[i] * d->OW + P.ph_oox[i]) * d->y_pitch;
-      const void* base = f32o ? (const void*)((const float*)d->y + off) : (const void*)((const bf16*)d->y + off);
-      rc = make_out_map(&P.ymap[i], base, f32o, d->Cout, P.ph_QW[i], P.ph_QH[i], d->N, (int64_t)d->osx * d->y_pitch,
+      const float* base = (const float*)d->y + ((int64_t)P.ph_ooy[i] * d->OW + P.ph_oox[i]) * d->y_pitch;
+      rc = make_out_map(&P.ymap[i], base, d->Cout, P.ph_QW[i], P.ph_QH[i], d->N, (int64_t)d->osx * d->y_pitch,
                         (int64_t)d->osy * d->OW * d->y_pitch, (int64_t)d->OH * d->OW * d->y_pitch, P.bw, P.bh, P.bn);
       if (rc) return rc;
     }
@@ -1541,17 +1297,10 @@ int conv_tc_launch(const bvae_conv_desc* d, cudaStream_t stream) {
   }
   const long grid = (long)P.tiles_w * P.tiles_h * P.tiles_n * P.n_tiles * P.nphase;
   BVAE_REQUIRE(grid > 0 && grid < (1l << 31), BVAE_ERR_SHAPE, "conv_tc: grid too large");
-  BVAE_REQUIRE(P.nphase == 1 || !use_conv_v1(), BVAE_ERR_UNSUPPORTED, "conv_tc: multi-phase needs the persistent kernel");
-  if (!use_conv_v1()) {
 #define CONV2_CASE(kb, bn) if (KB == kb && BN == bn) return launch_conv2<kb, bn>(P, grid, stream)
-    CONV2_CASE(64, 256); CONV2_CASE(64, 192); CONV2_CASE(64, 128); CONV2_CASE(64, 64); CONV2_CASE(64, 32);
-    CONV2_CASE(32, 256); CONV2_CASE(32, 192); CONV2_CASE(32, 128); CONV2_CASE(32, 64); CONV2_CASE(32, 32);
+  CONV2_CASE(64, 256); CONV2_CASE(64, 192); CONV2_CASE(64, 128); CONV2_CASE(64, 64); CONV2_CASE(64, 32);
+  CONV2_CASE(32, 256); CONV2_CASE(32, 192); CONV2_CASE(32, 128); CONV2_CASE(32, 64); CONV2_CASE(32, 32);
 #undef CONV2_CASE
-  }
-#define CONV_CASE(kb, bn, st) if (KB == kb && BN == bn) return launch_conv<kb, bn, st>(P, (int)grid, stream)
-  CONV_CASE(64, 256, 4); CONV_CASE(64, 192, 4); CONV_CASE(64, 128, 3); CONV_CASE(64, 64, 4); CONV_CASE(64, 32, 4);
-  CONV_CASE(32, 256, 4); CONV_CASE(32, 192, 4); CONV_CASE(32, 128, 4); CONV_CASE(32, 64, 4); CONV_CASE(32, 32, 4);
-#undef CONV_CASE
   set_error("conv_tc: no kernel for KB=%d BN=%d", KB, BN);
   return BVAE_ERR_UNSUPPORTED;
 }
@@ -1564,42 +1313,18 @@ int wgrad_tc_eligible(const bvae_wgrad_desc* d) {
   return plan_views(d->ntaps, d->dy, d->dx, d->sy, d->sx, &vp) ? 1 : 0;
 }
 
-template <int CB, int NS, int STAGES>
-static int launch_wgrad_mc(const WgradTcParams& P, int grid, cudaStream_t stream, int smem) {
-  static bool attr_done = false;
-  if (!attr_done) {
-    cudaError_t e = cudaFuncSetAttribute(wgrad_tc_kernel<CB, NS, STAGES, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem);
-    BVAE_REQUIRE(e == cudaSuccess, BVAE_ERR_CUDA, "wgrad_tc: cudaFuncSetAttribute(%d) failed: %s", smem, cudaGetErrorString(e));
-    attr_done = true;
-  }
-  cudaLaunchConfig_t cfg = {};
-  cfg.gridDim = dim3((unsigned)grid);
-  cfg.blockDim = dim3(128);
-  cfg.dynamicSmemBytes = smem;
-  cfg.stream = stream;
-  cudaLaunchAttribute attr[1];
-  attr[0].id = cudaLaunchAttributeClusterDimension;
-  attr[0].val.clusterDim.x = 2; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-  cfg.attrs = attr;
-  cfg.numAttrs = 1;
-  cudaError_t e = cudaLaunchKernelEx(&cfg, wgrad_tc_kernel<CB, NS, STAGES, true>, P);
-  BVAE_REQUIRE(e == cudaSuccess, BVAE_ERR_CUDA, "wgrad_tc: cluster launch failed: %s", cudaGetErrorString(e));
-  note_kernel("wgrad_tc_kernel<%d,%d,%d>+mc2", CB, NS, STAGES);
-  return check_launch("wgrad_tc");
-}
-
 constexpr int WT_RING_BUDGET = 200 * 1024;     // shared memory the WT ring may take (+ 2 KB of alignment / barriers)
 template <int NS, int STAGES>
-static int launch_wgrad_wt(const WgradTcParams& P, int grid, cudaStream_t stream, int /*smem of the fixed two-stage ring*/) {
+static int launch_wgrad_wt(const WgradTcParams& P, int grid, cudaStream_t stream) {
   const int smem = 1024 + 1024 + P.wt_stages * P.wt_stage_bytes;
   static bool attr_done = false;
   if (!attr_done) {
-    cudaError_t e = cudaFuncSetAttribute(wgrad_tc_kernel<64, NS, STAGES, false, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    cudaError_t e = cudaFuncSetAttribute(wgrad_tc_kernel<64, NS, STAGES, true>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          WT_RING_BUDGET + 2048);
     BVAE_REQUIRE(e == cudaSuccess, BVAE_ERR_CUDA, "wgrad_tc: cudaFuncSetAttribute failed: %s", cudaGetErrorString(e));
     attr_done = true;
   }
-  wgrad_tc_kernel<64, NS, STAGES, false, true><<<grid, 128, smem, stream>>>(P);
+  wgrad_tc_kernel<64, NS, STAGES, true><<<grid, 128, smem, stream>>>(P);
   note_kernel("wgrad_tc_kernel<64,%d,%d>+wt", NS, P.wt_stages);
   return check_launch("wgrad_tc");
 }
@@ -1614,27 +1339,19 @@ static int launch_wgrad(const WgradTcParams& P, int grid, cudaStream_t stream) {
     BVAE_REQUIRE(e == cudaSuccess, BVAE_ERR_CUDA, "wgrad_tc: cudaFuncSetAttribute(%d) failed: %s", smem, cudaGetErrorString(e));
     attr_done = true;
   }
-  if (P.mc == 2) {
-    if constexpr (CB == 64 && NS >= 128) return launch_wgrad_mc<CB, NS, STAGES>(P, grid, stream, smem);
-  }
   if (P.wt == 1) {
-    if constexpr (CB == 64) return launch_wgrad_wt<NS, STAGES>(P, grid, stream, smem);
+    if constexpr (CB == 64) return launch_wgrad_wt<NS, STAGES>(P, grid, stream);
   }
   wgrad_tc_kernel<CB, NS, STAGES><<<grid, 128, smem, stream>>>(P);
   note_kernel("wgrad_tc_kernel<%d,%d,%d>", CB, NS, STAGES);
   return check_launch("wgrad_tc");
 }
 
-// BVAE_WGRAD_HALO: 0 = off, 1 = on (default)
-static int wgrad_halo_mode() {
-  return option("BVAE_WGRAD_HALO", 1);
-}
-
 // acc_cols = accumulator columns a CTA drains in its epilogue (0: the halo kernel, which keeps the fill heuristic)
 static void wgrad_finish(const bvae_wgrad_desc* d, WgradTcParams* P, int out_tiles, bool* packed_, int acc_cols = 0) {
   const int max_splits = ceil_div(P->nchunks, 8);
   int splits = 1;
-  if (acc_cols > 0 && option("BVAE_WGRAD_SPLITS", 1) != 0) {
+  if (acc_cols > 0) {
     // Pixel splits from a cost model (round 3).  ncu on 512->512 3x3 at 6x4 x 512 bars (40 output tiles x 7 splits = 280 CTAs,
     // 28 chunks each, 85 us): a CTA spends only ~55 % of its 42 us in the K loop (0.8 us per 64-pixel chunk); zeroing the
     // ring, TMEM allocation, the pipeline fill and above all the epilogue -- 128 x 512 fp32 as vector atomics, not overlapped
@@ -1686,8 +1403,7 @@ static int wgrad_unpack(const bvae_wgrad_desc* d, cudaStream_t stream) {
 
 static int wgrad_halo_try(const bvae_wgrad_desc* d, const ViewPlan* vp, cudaStream_t stream, int* done) {
   *done = 0;
-  const int mode = wgrad_halo_mode();
-  if (mode == 0 || d->Ca != 64 || d->Cs != 64 || d->sy != 1 || d->sx != 1 || d->ntaps < 4 || d->ntaps > 16 || vp->nviews != 1)
+  if (d->Ca != 64 || d->Cs != 64 || d->sy != 1 || d->sx != 1 || d->ntaps < 4 || d->ntaps > 16 || vp->nviews != 1)
     return BVAE_OK;
   int dy0 = d->dy[0], dy1 = d->dy[0], dx0 = d->dx[0], dx1 = d->dx[0];
   for (int t = 1; t < d->ntaps; ++t) {
@@ -1767,9 +1483,8 @@ int wgrad_tc_launch(const bvae_wgrad_desc* d, cudaStream_t stream) {
     if (rc || done) return rc;
   }
   pick_box(d->N, d->AH, d->AW, 64, &P.bw, &P.bh, &P.bn);
-  const int mc_req = (option("BVAE_WGRAD_MC", 0) != 0 && CB == 64 && NS >= 128 && ceil_div(d->Ca, 128) % 2 == 0) ? 2 : 1;
-  // BVAE_WGRAD_WIDE_TMA (default 1): one 5-D TMA request per operand and tap (see wgrad_tc_kernel, WT)
-  const bool wt = CB == 64 && (P.bw * P.bh * P.bn) % 16 == 0 && mc_req == 1 && option("BVAE_WGRAD_WIDE_TMA", 1) != 0;
+  // one 5-D TMA request per operand and tap (see wgrad_tc_kernel, WT)
+  const bool wt = CB == 64 && (P.bw * P.bh * P.bn) % 16 == 0;
   P.wt = wt ? 1 : 0;
   const int a_atoms = d->Ca >= 128 ? 128 / CB : d->Ca / CB;
   int rc = wt ? make_view_map5(&P.amap, d->a, d->Ca, d->AW, d->AH, d->N, d->a_pitch, (int64_t)d->AW * d->a_pitch,
@@ -1793,12 +1508,9 @@ int wgrad_tc_launch(const bvae_wgrad_desc* d, cudaStream_t stream) {
   P.ntaps = d->ntaps; P.T = d->T;
   const int max_tpc = (512 / NS) > BVAE_MAX_TAPS ? BVAE_MAX_TAPS : (512 / NS);
   if (wt) {
-    // BVAE_WGRAD_STAGES (default 4): cap on the ring depth; 2 = the fixed ring of the other variants
     P.wt_stage_bytes = (128 / 64 + max_tpc * (NS / 64)) * (P.bw * P.bh * P.bn) * 128;
-    int nst = WT_RING_BUDGET / P.wt_stage_bytes, cap = option("BVAE_WGRAD_STAGES", 4);
-    if (cap < 2) cap = 2;
-    if (cap > 4) cap = 4;
-    P.wt_stages = nst > cap ? cap : (nst < 2 ? 2 : nst);
+    const int nst = WT_RING_BUDGET / P.wt_stage_bytes;
+    P.wt_stages = nst > 4 ? 4 : (nst < 2 ? 2 : nst);
   }
   P.tap_groups = ceil_div(d->ntaps, max_tpc);
   P.tpc = ceil_div(d->ntaps, P.tap_groups);
@@ -1807,11 +1519,6 @@ int wgrad_tc_launch(const bvae_wgrad_desc* d, cudaStream_t stream) {
   P.ra_tiles = ceil_div(d->Ca, 128); P.rs_tiles = d->Cs / NS;
   P.a_atoms = d->Ca >= 128 ? 128 / CB : d->Ca / CB;
   P.Ca = d->Ca; P.Cs = d->Cs;
-  // BVAE_WGRAD_MC=1 (opt-in): pairs of anchor tiles as 2-CTA clusters with the shifted tile multicast (>= 256 anchor
-  // channels).  Correct (parity-tested) but not faster -- 23 launches of <64,256,2> per step 3.98 ms at 0.47 of the tensor peak
-  // against 3.84 ms at 0.50 without: L2 is at a third of its throughput on these layers (ncu), so halving the L2 reads buys
-  // nothing, and the pair's lock-step (a stage is refilled only when both CTAs have consumed it) costs a little.
-  P.mc = mc_req;
 
   const int out_tiles = P.ra_tiles * P.rs_tiles * P.tap_groups;
   bool packed = false;
