@@ -311,6 +311,20 @@ int bvae_bar_score(const float* logits /* [bars][5760] */, const float* target /
                    int32_t* counts_out /* [bars][3] */, void* stream);
 
 /* ------------------------------------------------------------------------------------------------------------
+ * First and second moments of n latents of width d (row i at z + i*ld), accumulated in place in fp64 -- the statistics
+ * of the Gaussian prior fitted to the encoder's output (prior.py):
+ *   sum[j]     += sum_i z[i][j]
+ *   gram[j][k] += sum_i z[i][j] * z[i][k]      for k >= j; entries with k < j are neither read nor written
+ * Every product is formed in fp64 (exact for two fp32 values), and every output element adds its rows one at a time in
+ * increasing row order, starting from the value already in memory.  No atomics, no split of the rows across CTAs, no
+ * DMMA: a sequence of calls over consecutive chunks of rows gives the same bits as one call over all of them.
+ * n >= 0, d >= 1, ld >= d, else BVAE_ERR_SHAPE; z 4-byte and sum / gram 8-byte aligned, else BVAE_ERR_ALIGN.  n == 0
+ * writes nothing.
+ * ------------------------------------------------------------------------------------------------------------ */
+int bvae_latent_moments(const float* z /* [n][ld] */, int64_t n, int32_t d, int64_t ld, double* sum /* [d] */,
+                        double* gram /* [d][d] row-major */, void* stream);
+
+/* ------------------------------------------------------------------------------------------------------------
  * nn.BatchNorm2d(C, eps, momentum, affine) (+ optional (Leaky)ReLU) on an NHWC tensor with few channels: the norm of the
  * GAN-phase piano-roll discriminator (graph/bar_discriminator.py:19-23,69,113-114,153: BatchNorm2d(8..64, eps=1e-5,
  * momentum=0.01), OnOffFeature's default-momentum BatchNorm2d(8)) and of the Refiner (graph/refiner.py:13,20,37,43).

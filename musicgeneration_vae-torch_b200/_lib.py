@@ -118,6 +118,7 @@ SYMBOLS = [
     ("bvae_threshold_pack", C.c_int, [c_vp, c_i64, c_f32, c_vp, c_vp, c_vp]),
     ("bvae_bernoulli_sample", C.c_int, [c_vp, c_i64, c_f32, C.c_uint64, c_i64, c_i32, c_vp, c_vp]),
     ("bvae_bar_score", C.c_int, [c_vp, c_vp, c_i64, c_f32, c_f32, c_vp, c_vp, c_vp]),
+    ("bvae_latent_moments", C.c_int, [c_vp, c_i64, c_i32, c_i64, c_vp, c_vp, c_vp]),
     ("bvae_bn_scratch_floats", C.c_int, [C.c_int]),
     ("bvae_bn_forward", C.c_int, [C.POINTER(BnDesc), c_vp]),
     ("bvae_bn_backward", C.c_int, [C.POINTER(BnDesc), c_vp]),

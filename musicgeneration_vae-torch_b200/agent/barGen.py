@@ -246,9 +246,14 @@ class BarGen(object):
             self.logger.debug("pre_train lr: {}".format(self.lr_gen1))
         return avg_gen_loss.val
 
-    def generate(self, music_length=2, songs=1, seed=0, sampler="threshold", temperature=1.0, primer=None):
-        """per-epoch sample generation of agent/barGen2.py:316-336 (same loop as maker_bar.py)"""
+    def generate(self, music_length=2, songs=1, seed=0, sampler="threshold", temperature=1.0, primer=None,
+                 latent_prior=None):
+        """per-epoch sample generation of agent/barGen2.py:316-336 (same loop as maker_bar.py); ``latent_prior``
+        (prior.LatentPrior fitted to this generator's encoder) draws the latents instead of N(0, I)"""
         g = torch.Generator(device=self.device).manual_seed(seed)
-        lat = torch.randn(music_length * 4, songs, 1152, device=self.device, generator=g)
+        if latent_prior is not None:
+            lat = latent_prior.sample(music_length * 4, songs, g)
+        else:
+            lat = torch.randn(music_length * 4, songs, 1152, device=self.device, generator=g)
         return sample_songs(self.generator, lat, music_length, sampler=sampler, temperature=temperature,
                             seed=g.initial_seed(), primer=primer)

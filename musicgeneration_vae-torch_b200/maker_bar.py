@@ -8,7 +8,9 @@ Two extensions, both off by default: ``sampler="bernoulli"`` draws every cell fr
 distribution at a temperature instead of thresholding it (csrc/sample.cu), and ``primer`` continues given phrases
 instead of starting from silence."""
 import collections
+import itertools
 import math
+import os
 
 import numpy as np
 import torch
@@ -318,7 +320,12 @@ def main(argv=None):
     decode of those latents to ``--out`` and prints the teacher-forced score.  ``--interpolate a.mid b.mid`` encodes
     both files, cut to the same number of whole phrases (the smaller count, or ``--phrases``), and writes ``--steps``
     songs morphing from a to b: ``--out``, ``out_1``, ...  In both modes the song length is the file's, not
-    ``--music_length``."""
+    ``--music_length``.
+
+    ``--fit_prior OUT.pt --data SRC [SRC ...]`` fits a Gaussian to the checkpoint's latents of every bar of the sources
+    (``.mid`` files, whole phrases, or packed-array directories of ``tools/pack_dataset.py``), writes it to ``OUT.pt``
+    and samples nothing.  ``--latent_prior PRIOR.pt`` then draws the latents of the default and ``--primer`` modes from
+    that prior instead of N(0, I) (prior.py); a prior fitted to another checkpoint is refused."""
     import argparse
     from .graph.model import Model
     from .midi import write_midi
@@ -343,6 +350,12 @@ def main(argv=None):
     ap.add_argument("--phrases", type=int, default=None,
                     help="--reconstruct / --interpolate: phrases of the file(s) to use (default: the whole phrases "
                          "covered; for two files the smaller count)")
+    ap.add_argument("--latent_prior", default=None, metavar="PRIOR.pt",
+                    help="draw the latents from this fitted prior (--fit_prior) instead of N(0, I)")
+    ap.add_argument("--fit_prior", default=None, metavar="OUT.pt",
+                    help="fit a Gaussian prior to the checkpoint's latents of the --data bars, write it, sample nothing")
+    ap.add_argument("--data", nargs="+", default=None, metavar="SRC",
+                    help="--fit_prior: .mid files and packed-array directories (tools/pack_dataset.py) to fit on")
     args = ap.parse_args(argv)
     if not (math.isfinite(args.temperature) and args.temperature > 0):
         ap.error("--temperature must be finite and > 0")
@@ -362,6 +375,23 @@ def main(argv=None):
         ap.error("--phrases needs --reconstruct or --interpolate")
     if args.phrases is not None and args.phrases < 1:
         ap.error("--phrases must be at least 1")
+    if args.latent_prior is not None and encode_mode:
+        ap.error("--latent_prior does not apply to --%s" % encode_mode)
+    if args.fit_prior is not None:
+        if modes or args.latent_prior is not None:
+            ap.error("--fit_prior does not combine with --%s" % (modes[0] if modes else "latent_prior"))
+        if args.songs is not None:
+            ap.error("--songs does not apply to --fit_prior")
+        if args.data is None:
+            ap.error("--fit_prior needs --data")
+        for src in args.data:
+            if not (os.path.isfile(os.path.join(src, "note_bits.npy")) or
+                    (os.path.isfile(src) and src.lower().endswith((".mid", ".midi")))):
+                ap.error("--data %s is neither a .mid file nor a packed-array directory with note_bits.npy" % src)
+    elif args.data is not None:
+        ap.error("--data needs --fit_prior")
+    if args.latent_prior is not None and not os.path.isfile(args.latent_prior):
+        ap.error("--latent_prior %s: no such file" % args.latent_prior)
     primer = None
     if args.primer is not None:
         try:
@@ -381,6 +411,25 @@ def main(argv=None):
         rolls_in = np.stack([r[:P * PHRASE_STEPS] for r in rolls_in])
     dev = torch.device("cuda", torch.cuda.current_device())
     model = load_generator(Model().to(dev), "model/checkpoint_{}.pth.tar".format(args.model_number), dev)
+    if args.fit_prior is not None:
+        from .prior import bars_of_midi, bars_of_packed, fit_latent_prior, save_latent_prior
+        srcs = [bars_of_packed(src) if os.path.isdir(src) else bars_of_midi([src]) for src in args.data]
+        try:
+            prior = fit_latent_prior(model, itertools.chain.from_iterable(srcs))
+        except ValueError as e:
+            ap.error(str(e))
+        save_latent_prior(prior, args.fit_prior)
+        print("latent prior: %d bars, |mean| %.6g, sqrt(trace(cov) / d) %.6g, shrinkage %g -> %s"
+              % (prior.count, float(prior.mean.norm()), math.sqrt(float(torch.trace(prior.cov)) / prior.dim),
+                 prior.shrinkage, args.fit_prior))
+        return
+    prior = None
+    if args.latent_prior is not None:
+        from .prior import load_latent_prior
+        try:
+            prior = load_latent_prior(args.latent_prior, model)
+        except ValueError as e:
+            ap.error(str(e))
     g = torch.Generator(device=dev)
     if args.seed is not None:
         g.manual_seed(args.seed)
@@ -394,6 +443,8 @@ def main(argv=None):
     elif encode_mode == "interpolate":
         z = encode_songs(model, rolls_in)
         lat, length = interpolate_latents(z[:, 0], z[:, 1], 5 if args.steps is None else args.steps), P
+    elif prior is not None:
+        lat = prior.sample(args.music_length * 4, 1 if args.songs is None else args.songs, g)
     else:
         lat = torch.randn(args.music_length * 4, 1 if args.songs is None else args.songs, 1152, device=dev,
                           generator=g)
